@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 5            # this repo's CUDA engine
     python bench.py --impl reference --gpus 1 --steps 3 --warmup 2   # CPU reference path (oracle port)
     python bench.py --workload resnet18_iao_w8a8_bnfuse       # another BASELINE.json config as the measured workload
+    python bench.py --steps 20 --dump-outputs DIR             # + what the last timed step computed, as DIR/<name>.npy
 
 Workload (BASELINE.json configs[1]): NIN-GC, wbwtab W-ternary / A-binary, batch 256 per GPU,
 3x32x32 inputs, CrossEntropy + Adam(lr 0.01) - the reference's training step
@@ -24,6 +25,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -35,6 +37,7 @@ from harness import train as H  # noqa: E402
 WORKLOAD = "nin_gc_wbwtab_w3a2"   # BASELINE.json configs[1]; --workload picks another config
 BATCH_PER_GPU = 256
 CPU_SAMPLE_BATCH = 32
+DUMP_BYTES = 64 * 10**6   # --dump-outputs budget, .npy headers included
 NAMES = {"nin_gc_wbwtab_w3a2": "NIN-GC wbwtab W-ternary/A-binary QAT step (BASELINE.json configs[1])",
          "nin_dorefa_w8a8": "NIN DoReFa W8A8 QAT step (configs[0] model)",
          "resnet18_iao_w8a8_bnfuse": "ResNet-18 IAO W8A8 per-channel + BN-fuse QAT step (configs[2])",
@@ -198,8 +201,34 @@ def main_reference(args):
 # ----------------------------------------------------------------------------------------------------------
 # engine arm
 # ----------------------------------------------------------------------------------------------------------
-def run_engine(workload, steps, warmup, dev, rank, world, detail):
-    """time `steps` steps of one workload; returns the measurement dict (rank-local, max over ranks for times)"""
+def dump_outputs(path, model, result, inference):
+    """write what the last timed step handed its caller as <path>/<name>.npy (float32): the logits of an inference
+    step; the loss of a QAT step with the parameters and floating-point buffers it updated and the gradients it
+    computed.  Past DUMP_BYTES in all, every array is cut to the same fraction of its elements, a seeded random
+    sample kept in index order (flattened), so that two builds fed the same arguments dump comparable arrays."""
+    arrays = {"logits" if inference else "loss": result}
+    if not inference:
+        for n, p in model.named_parameters():
+            arrays[f"param.{n}"] = p
+            if p.grad is not None:
+                arrays[f"grad.{n}"] = p.grad
+        for n, b in model.named_buffers():
+            if b.is_floating_point():
+                arrays[f"buffer.{n}"] = b
+    total = sum(a.numel() for a in arrays.values())
+    keep = min(1.0, (DUMP_BYTES - 256 * len(arrays)) / 4 / total)   # 256 B: the header of one .npy file, and its one kept element
+    os.makedirs(path, exist_ok=True)
+    for i, (name, a) in enumerate(arrays.items()):
+        a = a.detach().float().cpu()
+        if keep < 1.0:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(i))[:max(1, int(a.numel() * keep))]
+            a = a.flatten()[idx.sort().values]
+        np.save(os.path.join(path, f"{name}.npy"), a.numpy())
+
+
+def run_engine(workload, steps, warmup, dev, rank, world, detail, dump=None):
+    """time `steps` steps of one workload; returns the measurement dict (rank-local, max over ranks for times).
+    `dump`: directory that receives what the last timed step computed (rank 0)"""
     from micronet_b200 import _lib as L, functional as F_
     w = H.WORKLOADS[workload]
     inference = bool(w.get("inference"))
@@ -233,9 +262,11 @@ def run_engine(workload, steps, warmup, dev, rank, world, detail):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return ms.item()
 
+    last = [None]
+
     def step_resident(i):
         x, t = devb[i % nbuf]
-        stepper.step(x, t)
+        last[0] = stepper.step(x, t).detach()   # a loss kept with its autograd graph would break the CUDA graph capture
 
     out_host = torch.empty((B, 10) if inference else (), dtype=torch.float32).pin_memory()
 
@@ -257,6 +288,8 @@ def run_engine(workload, steps, warmup, dev, rank, world, detail):
     torch.cuda.synchronize()
     L.tc_check()   # a bounded pipeline wait that gave up would have produced garbage: fail loudly instead
     clocks = sampler.stop() if sampler else None
+    if dump and rank == 0:
+        dump_outputs(dump, model, last[0], inference)
     for i in range(2):
         step_e2e(i)
     ms_e2e = timed(step_e2e, steps)
@@ -323,7 +356,11 @@ def main():
     ap.add_argument("--kernels-json", default=None, help="dump the per-kernel CUDA-event timings of the timed region")
     ap.add_argument("--workload", default=WORKLOAD, choices=sorted(H.WORKLOADS),
                     help="default: the headline configuration (BASELINE.json configs[1])")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step of the workload computed to DIR/<name>.npy (float32, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return main_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -342,7 +379,7 @@ def main():
     torch.backends.cuda.matmul.allow_tf32 = False
 
     wl = args.workload
-    main_res = run_engine(wl, args.steps, args.warmup, dev, rank, world, detail=True)
+    main_res = run_engine(wl, args.steps, args.warmup, dev, rank, world, detail=True, dump=args.dump_outputs)
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()

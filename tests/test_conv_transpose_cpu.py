@@ -1,16 +1,14 @@
-"""`QuantConvTranspose2d` on the CPU side (SURVEY 8 row f4): module surface / prepare() of all three schemes without a GPU, and -
-where the reference tree is present (build container only) - the evidence that the reference's OWN wbwtab / dorefa classes are
-not runnable under current PyTorch, which is why only the IAO one (IAO:510-636) has golden fixtures generated from the reference
+"""`QuantConvTranspose2d` on the CPU side (SURVEY 8 row f4): module surface / prepare() of all three schemes without a GPU, and
+the evidence, recorded from the reference, that the reference's OWN wbwtab / dorefa classes are not runnable under current
+PyTorch, which is why only the IAO one (IAO:510-636) has golden fixtures generated from the reference
 (tests/golden/layer_iao_convT_*.npz) and the other two are pinned on the oracle's quantizers composed with ATen."""
 import copy
-import os
-import sys
 
 import pytest
 import torch
 import torch.nn as nn
 
-REF = os.environ.get("MICRONET_REFERENCE", "/root/reference")
+from tests.oracle_util import load_golden, rel_err
 
 
 def _net():
@@ -42,21 +40,24 @@ def test_prepare_swaps_conv_transpose_in_every_scheme():
             m(torch.randn(1, 16, 4, 4))
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "micronet")), reason="reference tree not present (GPU box)")
 def test_reference_dorefa_and_wbwtab_conv_transpose_do_not_run():
-    sys.path.insert(0, REF)
-    try:
-        import micronet.compression.quantization.wbwtab.quantize as ref_wb
-        import micronet.compression.quantization.wqaq.dorefa.quantize as ref_df
-        import micronet.compression.quantization.wqaq.iao.quantize as ref_iao
-    finally:
-        sys.path.remove(REF)
-    x = torch.randn(2, 8, 5, 5)
-    m = ref_df.QuantConvTranspose2d(8, 6, 3, stride=2, padding=1, output_padding=1)
-    assert m.dilation == (True, True)          # `bias` landed in `dilation` (DF:142-153 vs nn.ConvTranspose2d's argument order)
-    with pytest.raises(TypeError):
-        m(x)
-    with pytest.raises(TypeError):
-        ref_wb.QuantConvTranspose2d(8, 6, 3, stride=2, padding=1, output_padding=1)(x)
-    y = ref_iao.QuantConvTranspose2d(8, 6, 3, stride=2, padding=1, output_padding=1)(x)   # keyword-correct: runs
+    """what the reference's own classes did for QuantConvTranspose2d(8, 6, 3, stride=2, padding=1, output_padding=1),
+    recorded by tests/golden/make_golden_convT_reference.py"""
+    from micronet_b200 import dorefa, wbwtab
+    from oracle import reference_port as O
+    gold = load_golden("reference", "convT_modules")
+    assert tuple(gold["dorefa.dilation"]) == (True, True)   # `bias` landed in `dilation` (DF:142-153 vs nn.ConvTranspose2d's argument order)
+    for scheme in ("dorefa", "wbwtab"):
+        err = str(gold[f"{scheme}.error"])
+        assert err.startswith("TypeError") and "dilation" in err, err
+    # the engine's modules take the same call with the geometry the reference meant
+    for m in (dorefa.QuantConvTranspose2d(8, 6, 3, stride=2, padding=1, output_padding=1),
+              wbwtab.QuantConvTranspose2d(8, 6, 3, stride=2, padding=1, output_padding=1)):
+        assert m.dilation == (1, 1) and m.groups == 1 and m.bias is not None
+        assert m.stride == (2, 2) and m.padding == (1, 1) and m.output_padding == (1, 1)
+    # the IAO class is keyword-correct and runs: the oracle port reproduces its output
+    iao = O.IaoQuantConvTranspose2d(8, 6, 3, stride=2, padding=1, output_padding=1)
+    iao.load_state_dict({k[len("iao.init."):]: torch.from_numpy(v) for k, v in gold.items() if k.startswith("iao.init.")})
+    y = iao(torch.from_numpy(gold["x"]))
     assert tuple(y.shape) == (2, 6, 10, 10)
+    assert rel_err(y.detach(), gold["iao.y"]) <= 1e-6

@@ -73,18 +73,3 @@ def test_tma_box_and_oob_fill(coord, tmp_path):
     out = subprocess.run([sys.executable, str(script), root, *map(str, coord)], capture_output=True, text=True,
                          timeout=300)
     assert out.returncode == 0 and "TMA_OK" in out.stdout, out.stdout[-2000:] + out.stderr[-2000:]
-
-
-@pytest.mark.parametrize("coord", [(3, 2, 1), (-2, -1, 0)], ids=str)
-def test_tma_unaligned_inner_coordinate_probe(coord, tmp_path):
-    """documents (does not require) what the hardware does when the innermost start coordinate is
-    not a multiple of 16 bytes; the conv kernels never rely on it."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    script = tmp_path / "tma_case.py"
-    script.write_text(TMA_CASE)
-    out = subprocess.run([sys.executable, str(script), root, *map(str, coord)], capture_output=True, text=True,
-                         timeout=300)
-    print("unaligned-inner probe", coord, "->", "ok" if "TMA_OK" in out.stdout else "faults / differs")
