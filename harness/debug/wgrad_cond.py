@@ -27,7 +27,7 @@ def run(name, B, C, H, K, R, G, kind):
     TF.conv2d(x, w32, None, 1, R // 2, 1, G).backward(go)
     cond = (TF.conv2d(x.abs().double().transpose(0, 1), go.abs().double().transpose(0, 1)[:K // G], None, 1, R // 2).max() / wr.grad.abs().max()).item() if G == 1 else float("nan")
     out = {}
-    for tag, env in (("tc", {}), ("pk3", {"pk": 3}), ("pk2", {"pk": 2})):
+    for tag, env in (("auto", {}), ("pk3", {"pk": 3}), ("pk2", {"pk": 2})):
         wg = wq.to(DEV).requires_grad_(True)
         if "pk" in env:
             L.PK_MODE, L.PK_TERMS_BWD = "all", env["pk"]

@@ -1,5 +1,6 @@
 """debug: weight gradient of one wbwtab layer on the REAL tensors of a golden model step (oracle capture), through the
-fused tensor-core kernel, the packed-operand kernel and the CUDA-core kernel, each against an fp64 replay."""
+default dispatch, the packed-operand kernel with 3 and 2 gradient pieces and the CUDA-core kernel, each against an fp64
+replay."""
 import copy, sys
 import torch
 from tests.golden.cases import MODEL_CASES
@@ -34,7 +35,7 @@ for n, c in cap.items():
     xo = xi.double().clone().requires_grad_(True)
     o64(xo).backward(go.double())
     ref = o64.weight.grad
-    for tag, setup in (("fused-tc", dict()), ("generic", dict(USE_TC=False, PK_MODE="off")), ("pk3", dict(PK_MODE="all", PK_TERMS_BWD=3)), ("pk2", dict(PK_MODE="all", PK_TERMS_BWD=2))):
+    for tag, setup in (("default", dict()), ("generic", dict(PK_MODE="off")), ("pk3", dict(PK_MODE="all", PK_TERMS_BWD=3)), ("pk2", dict(PK_MODE="all", PK_TERMS_BWD=2))):
         saved = {k: getattr(L, k) for k in setup}
         for k, v in setup.items(): setattr(L, k, v)
         try:
@@ -48,5 +49,5 @@ for n, c in cap.items():
     s = 1.0 / go.abs().max()
     e = copy.deepcopy(dict(em.named_modules())[n]); xe = xi.to(DEV).requires_grad_(True)
     e(xe).backward((go * s).to(DEV))
-    print(f"   fused-tc with go scaled to max 1: dW vs f64 {rel_err(e.weight.grad / s, ref):.2e}")
+    print(f"   default with go scaled to max 1: dW vs f64 {rel_err(e.weight.grad / s, ref):.2e}")
 L.tc_check()

@@ -186,42 +186,6 @@ int mnb_channel_stats(const float* x, int32_t batch, int32_t channels, int32_t h
 int mnb_channel_stats_bwd(const float* x, const float* mean, const float* dmean, const float* dvar,
                           int32_t batch, int32_t channels, int32_t hw, float* dx, mnb_stream_t stream);
 
-/* ------------------------------------------------------------------------
- * Fused tensor-core forward (tcgen05 + TMA): fake-quantize the fp32 NCHW input on the fly while
- * it is staged for the MMA, convolve exact integer levels, scale + bias in the epilogue.
- *   qp == NULL : x is used as it is (wbwtab: +-1 or plain fp32 activations, exact 3-term bf16 split)
- *   qp != NULL : DoReFa / IAO quantizer; `codes` (u8, same shape as x) and `pass_bits`
- *                (u32[ceil(numel/32)], ZERO-INITIALISED by the caller) receive what backward needs.
- * Replaces activation_quantizer(input) + F.conv2d of DF:108-121 / IAO:493-506 / WB:186-194.
- * Returns MNB_E_UNSUPPORTED (and launches nothing) for geometries outside the kernel's cover
- * (see mnb_conv_tc.cu); the caller then composes mnb_act_quant_fwd + mnb_conv2d_fwd.
- * err_flag: device int, stays 0 unless a bounded pipeline wait timed out (a bug, never expected).
- * ---------------------------------------------------------------------- */
-int mnb_fq_conv2d_fwd_tc(const mnb_conv_shape* s, const float* x, const mnb_act_qparams* qp,
-                         const int16_t* w_int, const float* w_scale, const float* bias, float* y,
-                         uint8_t* codes, uint32_t* pass_bits, void* wpack_scratch, int32_t* err_flag,
-                         mnb_stream_t stream);
-/* wpack_scratch: >= 2 * numel(w_int) bytes, 16-byte aligned (bf16 operand image of the weights). */
-
-/* Data gradient of the same convolution on the tensor-core path (ATen convolution_backward's
- * grad_input): dx = STE( conv_transpose(dy, w_scale[k] * w_int) ), the per-channel weight scale folded
- * into dy while it is staged (exact 3-term bf16 split of the fp32 product).  pass_bits / qp NULL:
- * plain dgrad (wbwtab).  Same geometry cover and error conventions as mnb_fq_conv2d_fwd_tc.   */
-int mnb_conv2d_dgrad_tc(const mnb_conv_shape* s, const float* dy, const int16_t* w_int, const float* w_scale,
-                        const uint32_t* pass_bits, const mnb_act_qparams* qp, float* dx, void* wpack_scratch,
-                        int32_t* err_flag, mnb_stream_t stream);
-
-/* Weight gradient on the tensor-core path: dWq = s_a * corr(e_a, dy) with e_a re-quantized from the
- * fp32 input x on the fly (qp as in the forward; NULL = raw x, which must be bf16-exact such as the
- * +-1 activations of wbwtab - otherwise *inexact_flag is set on the device and the result is to be
- * replaced by mnb_conv2d_wgrad_cond(..., inexact_flag), which runs only when the flag is non-zero,
- * so no host synchronisation is needed).  scratch >= mnb_wgrad_tc_scratch_bytes(s) (-1: unsupported). */
-int64_t mnb_wgrad_tc_scratch_bytes(const mnb_conv_shape* s);
-int mnb_conv2d_wgrad_tc(const mnb_conv_shape* s, const float* dy, const float* x, const mnb_act_qparams* qp,
-                        float* dwq, void* scratch, int32_t* inexact_flag, int32_t* err_flag, mnb_stream_t stream);
-int mnb_conv2d_wgrad_cond(const mnb_conv_shape* s, const float* dy, const mnb_conv_operands* op, float* dwq,
-                          void* scratch, const int32_t* run_if_nonzero, mnb_stream_t stream);
-
 /* Producer-side fusions of a wbwtab block (SURVEY.md 8 f2):
  *   conv -> nn.BatchNorm2d -> ActivationQuantizer(A=2) [-> nn.MaxPool2d] -> channel_shuffle -> next conv
  * (nin_gc.py:9-21 shuffle, :53-59 block, WB:79-94 binarizer).
@@ -401,10 +365,6 @@ int mnb_xnor_conv_fwd(const mnb_conv_shape* s, const void* a_bits, const void* w
  * wbwtab/main.py:84,331-339) over one flat fp32 parameter / gradient bucket: a single launch. */
 int mnb_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n, float lr,
                   float beta1, float beta2, float eps, float weight_decay, int32_t step, mnb_stream_t stream);
-
-/* Debug hook: 16 int64 device counters [role: tma, mma, epilogue, converter][wait a, wait b, wait c,
- * total cycles], accumulated by the fwd/dgrad tensor-core kernel while the pointer is non-NULL.  */
-void mnb_set_tc_profile_buffer(void* dev_int64x16);
 
 /* ------------------------------------------------------------------------
  * Hardware self-tests of the sm_100a building blocks (run by tests/test_gpu_tc_selftest.py).

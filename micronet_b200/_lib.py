@@ -68,11 +68,6 @@ PROTOTYPES = {
     "mnb_conv2d_wgrad": (C.c_int, [_SHAPE, _P, _OPS, _P, _P, _P]),
     "mnb_channel_stats": (C.c_int, [_P, _I, _I, _I, _I, _P, _P, _P]),
     "mnb_channel_stats_bwd": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _P, _P]),
-    "mnb_fq_conv2d_fwd_tc": (C.c_int, [_SHAPE, _P, _ACTQ, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
-    "mnb_conv2d_dgrad_tc": (C.c_int, [_SHAPE, _P, _P, _P, _P, _ACTQ, _P, _P, _P, _P]),
-    "mnb_wgrad_tc_scratch_bytes": (_L, [_SHAPE]),
-    "mnb_conv2d_wgrad_tc": (C.c_int, [_SHAPE, _P, _P, _ACTQ, _P, _P, _P, _P, _P]),
-    "mnb_conv2d_wgrad_cond": (C.c_int, [_SHAPE, _P, _OPS, _P, _P, _P, _P]),
     "mnb_bn_batch_stats": (C.c_int, [_P, _I, _I, _I, _D, _D, _P, _P, _P, _P, _P, _P]),
     "mnb_bn_sign_fwd": (C.c_int, [_P, _I, _I, _I, _P, _P, _P, _P, _I, _P, _P, _P]),
     "mnb_bn_sign_bwd": (C.c_int, [_P, _P, _P, _I, _I, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P]),
@@ -105,7 +100,6 @@ PROTOTYPES = {
     "mnb_xnor_wimage_bytes": (_L, [_SHAPE]),
     "mnb_xnor_pack_weight": (C.c_int, [_SHAPE, _P, _P, _P]),
     "mnb_xnor_conv_fwd": (C.c_int, [_SHAPE, _P, _P, _P, _P, _P, _P]),
-    "mnb_set_tc_profile_buffer": (None, [_P]),
     "mnb_selftest_mma_rate": (C.c_int, [_I, _I, _I, _I, _I, _P, _P, _P]),
     "mnb_selftest_umma": (C.c_int, [_P, _P, _P, _I, _I, _I, _P, _P]),
     "mnb_selftest_tma3d": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int32), C.POINTER(C.c_int32), _P, _P, _P]),
@@ -186,13 +180,9 @@ def tc_check(device=None):
 
 E_UNSUPPORTED = -2
 KEEP_DEBUG = False   # tests only: modules keep the fake-quantized weight of their last call
-USE_TC = os.environ.get("MNB_DISABLE_TC", "0") != "1"
-# packed bf16 operands from the BN+binarizer producer to the next conv's forward.  Measured (r2h): the convs gain 0.1 ms per
-# step (fwd 158 -> 120 us on the 256-channel 1x1) but the producer's extra 2 B / element plane and its scalar form cost 0.7 ms,
-# so it stays opt-in (MNB_PACKED_OPERANDS=1) until the producer is vectorised and stops writing the fp32 plane as well
-USE_PACKED = os.environ.get("MNB_PACKED_OPERANDS", "0") == "1"
-# packed-operand tensor-core family (mnb_pk.cu): "auto" = wherever the fused kernels have no cover and for every fused-quantizer
-# layer; "all" = every conv it supports; "off" = never
+# packed-operand tensor-core family (mnb_pk.cu): "auto" = every fused-quantizer layer, every conv behind a binarizer and every
+# conv the fp32 first-layer kernels (mnb_conv_fp32_tc.cu) do not take; "all" = every conv it supports, before those kernels;
+# "off" = never (the generic kernels then run every conv: the reference arm of the tests)
 PK_MODE = os.environ.get("MNB_PK", "auto")
 # exact bf16 pieces per fp32 operand on the pk path (3 = exact 24-bit split; 2 = 16 bits, ~4e-6 relative)
 PK_TERMS = int(os.environ.get("MNB_PK_TERMS", "3"))
@@ -202,10 +192,6 @@ PK_TERMS = int(os.environ.get("MNB_PK_TERMS", "3"))
 # decides an integer level depends on them.  The forward statistics conv keeps PK_TERMS (its mean / variance decide the
 # quantized weight levels).  MNB_PK_TERMS_BWD=3 restores the exact split.
 PK_TERMS_BWD = int(os.environ.get("MNB_PK_TERMS_BWD", "2"))
-# wbwtab layers between two fused BatchNorm + binarizer producers (fused.BatchNormBinarize2d) take the packed-operand family
-# with BOTH operands written by the producers: +-1 planes forward (mnb_bn_sign_fwd_packed), gradient pieces backward
-# (mnb_bn_sign_bwd_pack); 3x3 layers take it in any case.  MNB_PK_WBWTAB=0 keeps every wbwtab layer on the fused kernels.
-PK_WBWTAB = os.environ.get("MNB_PK_WBWTAB", "1") == "1"
 
 # bit-packed XNOR-popcount forward for wbwtab inference (mnb_xnor.cu): "auto" = the layers where it was measured to beat the
 # tensor-core forward (functional.xnor_preferred), "all" = wherever it has cover, "off" = never

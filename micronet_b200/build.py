@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libmicronet_b200.so")
-SOURCES = ["mnb_quant.cu", "mnb_fused.cu", "mnb_conv_generic.cu", "mnb_conv_tc.cu", "mnb_conv_tc_fwd.cu", "mnb_conv_tc_wgrad.cu", "mnb_conv_fp32_tc.cu", "mnb_conv_packed.cu", "mnb_pk.cu", "mnb_xnor.cu"]
+SOURCES = ["mnb_quant.cu", "mnb_fused.cu", "mnb_conv_generic.cu", "mnb_conv_tc.cu", "mnb_conv_fp32_tc.cu", "mnb_conv_packed.cu", "mnb_pk.cu", "mnb_xnor.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -1,8 +1,8 @@
 // fp32 convolution with few input channels (the un-quantized FIRST layer of every QAT model: 3 -> 192/256,
 // 5x5 or 3x3; nin_gc.py:82, nin.py, resnet.py) on tcgen05 tensor cores: forward and weight gradient.
 //
-// C*R*S (75 for 3x5x5) is far too small a reduction for the per-tap implicit GEMM of mnb_conv_tc_fwd.cu
-// (one MMA K-step would carry 3 real channels out of 16), so this layer uses a real im2col operand, built in
+// C*R*S (75 for 3x5x5) is far too small a reduction for a per-tap implicit GEMM (one MMA K-step would carry 3
+// real channels out of 16), so this layer uses a real im2col operand, built in
 // shared memory from a zero-padded input patch:
 //
 //   forward : y[b, n, pos]  = bias[n] + sum_kk  Xcol[pos, kk] * w[n, kk]      M = 128 positions, N = Cout, K = kk

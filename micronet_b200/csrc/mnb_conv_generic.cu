@@ -3,7 +3,7 @@
 // This is the shape-agnostic path of the engine: forward (exact s32 accumulation when both
 // operands are integer levels, fp32 otherwise), dgrad fused with the activation STE mask, and
 // split-K wgrad with a deterministic two-stage reduction.  Hot, regular shapes are taken by the
-// tcgen05 tensor-core kernels in mnb_conv_tc.cu; everything else (C_in = 3 stems, 10-way heads,
+// tcgen05 tensor-core kernels in mnb_pk.cu and mnb_conv_fp32_tc.cu; everything else (C_in = 3 stems, 10-way heads,
 // odd strides, asymmetric weights) lands here.
 //
 // GEMM views (per group g; Cg = in_c/groups, Ng = out_c/groups, RS = kh*kw):
@@ -253,7 +253,6 @@ struct WgradArgs {
   const float* dy; const uint8_t* a_codes; const float* a_f32; int a_off; const float* a_off_zp;
   float* partial;  // [splits][out_c * Cg * RS]
   int splits, k_per_split;
-  const int* run_if;  // optional device flag: the kernels return immediately when *run_if == 0
 };
 
 template <int BN>
@@ -261,7 +260,6 @@ __global__ void __launch_bounds__(NT) conv_wgrad_kernel(WgradArgs a) {
   constexpr int TN = BN / 16;
   __shared__ float As[BK][BM + 1];
   __shared__ float Bs[BK][BN + 1];
-  if (a.run_if && *a.run_if == 0) return;
   const ConvGeom& g = a.g;
   const int grp = blockIdx.z / a.splits, split = blockIdx.z - grp * a.splits;
   const int m0 = blockIdx.x * BM, n0 = blockIdx.y * BN;
@@ -343,8 +341,7 @@ __global__ void __launch_bounds__(NT) conv_wgrad_kernel(WgradArgs a) {
 
 __global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float* __restrict__ partial, int64_t n,
                                                            int splits, const float* a_scale,
-                                                           float* __restrict__ dwq, const int* run_if) {
-  if (run_if && *run_if == 0) return;
+                                                           float* __restrict__ dwq) {
   const float sc = a_scale ? __ldg(a_scale) : 1.f;
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -430,24 +427,9 @@ extern "C" int64_t mnb_wgrad_scratch_bytes(const mnb_conv_shape* s) {
   return (int64_t)splits * g.K * g.Cg * g.RS * 4;
 }
 
-static int wgrad_impl(const mnb_conv_shape* s, const float* dy, const mnb_conv_operands* op, float* dwq,
-                      void* scratch, const int32_t* run_if, mnb_stream_t stream);
-
 extern "C" int mnb_conv2d_wgrad(const mnb_conv_shape* s, const float* dy, const mnb_conv_operands* op,
                                 float* dwq, void* scratch, mnb_stream_t stream) {
-  return wgrad_impl(s, dy, op, dwq, scratch, nullptr, stream);
-}
-extern "C" int mnb_conv2d_wgrad_cond(const mnb_conv_shape* s, const float* dy, const mnb_conv_operands* op,
-                                     float* dwq, void* scratch, const int32_t* run_if_nonzero,
-                                     mnb_stream_t stream) {
-  MNB_REQUIRE(run_if_nonzero != nullptr, "run_if_nonzero is NULL");
-  return wgrad_impl(s, dy, op, dwq, scratch, run_if_nonzero, stream);
-}
-
-static int wgrad_impl(const mnb_conv_shape* s, const float* dy, const mnb_conv_operands* op, float* dwq,
-                      void* scratch, const int32_t* run_if, mnb_stream_t stream) {
   WgradArgs a;
-  a.run_if = run_if;
   if (int e = make_geom(s, a.g)) return e;
   MNB_REQUIRE(dy && op && dwq && scratch, "NULL wgrad pointers");
   MNB_REQUIRE((op->a_codes != nullptr) != (op->a_f32 != nullptr), "exactly one of a_codes / a_f32 must be given");
@@ -465,7 +447,7 @@ static int wgrad_impl(const mnb_conv_shape* s, const float* dy, const mnb_conv_o
   else conv_wgrad_kernel<64><<<grid, NT, 0, st>>>(a);
   const int64_t n = (int64_t)g.K * Nd;
   int blocks = (int)std::min<int64_t>(mnb_ceil_div(n, 256), MNB_NUM_SMS * 8);
-  wgrad_reduce_kernel<<<blocks, 256, 0, st>>>(a.partial, n, a.splits, op->a_codes ? op->a_scale : nullptr, dwq, run_if);
+  wgrad_reduce_kernel<<<blocks, 256, 0, st>>>(a.partial, n, a.splits, op->a_codes ? op->a_scale : nullptr, dwq);
   MNB_LAUNCHED(2);
   return 0;
 }

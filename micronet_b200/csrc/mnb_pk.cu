@@ -1,10 +1,9 @@
 // Packed-operand ("pk") tensor-core convolution family: any conv geometry of the QAT models on tcgen05.
 //
-// Why a second family next to mnb_conv_tc_fwd.cu / mnb_conv_tc_wgrad.cu: those kernels keep the whole weight
-// slab of a group resident in shared memory and convert fp32 activations inside the kernel, which limits them
-// to small grouped layers (NIN-GC).  ResNet-18 (up to 512 -> 512 3x3 = 9.4 MB of weights, stride 2, 4x4 images),
-// NIN's 5x5 96 -> 192 and 224x224 inputs need the B operand STREAMED and N / W tiling.  Here every operand
-// reaches the kernel already in the layout the tensor core reads:
+// ResNet-18 (up to 512 -> 512 3x3 = 9.4 MB of weights, stride 2, 4x4 images), NIN's 5x5 96 -> 192 and 224x224
+// inputs need the B operand STREAMED and N / W tiling, so no weight slab stays resident in shared memory and no
+// kernel converts fp32 activations itself.  Every operand reaches the kernel already in the layout the tensor core
+// reads:
 //
 //   activations / gradients : bf16 "term planes"  pk[t][b][c/8][h][w][8]   (16 bytes = 8 channels of one pixel)
 //                             t = 0 .. T-1 exact pieces of an fp32 value (x = p0 + p1 + p2, 8 significand bits each)

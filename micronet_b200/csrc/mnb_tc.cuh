@@ -95,15 +95,6 @@ __device__ __forceinline__ void tma_load_4d(void* smem_dst, const CUtensorMap* m
       : "memory");
 }
 
-__device__ __forceinline__ void tma_load_5d(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1,
-                                            int c2, int c3, int c4) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cta.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2),
-      "r"(c3), "r"(c4)
-      : "memory");
-}
-
 // plain 1-D bulk copy global -> shared (size multiple of 16 bytes), completion on an mbarrier
 __device__ __forceinline__ void bulk_load_1d(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
@@ -146,35 +137,11 @@ __device__ __forceinline__ void mma_f16_guarded(uint32_t d_tmem, uint64_t adesc,
       ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"(guard)
       : "memory");
 }
-// Same, descriptors given as (low word, high word): only the 14-bit start-address field of the low word changes from
-// MMA to MMA, so issue loops carry 32-bit adds and the loop-invariant high words stay in uniform registers.
-__device__ __forceinline__ void mma_f16_guarded_lh(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo,
-                                                   uint32_t b_hi, uint32_t idesc, uint32_t accumulate, uint32_t guard) {
-  asm volatile(
-      "{\n\t.reg .pred p, q;\n\t.reg .b64 da, db;\n\t"
-      "setp.ne.b32 p, %6, 0;\n\tsetp.ne.b32 q, %7, 0;\n\t"
-      "mov.b64 da, {%1, %2};\n\tmov.b64 db, {%3, %4};\n\t"
-      "@q tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n\t}"
-      ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate), "r"(guard)
-      : "memory");
-}
-// Warp-converged issue with the hardware election inside the instruction group: `elect.sync` tells ptxas that exactly
-// one lane issues, so no per-lane ELECT / BRA.U.ANY loop is generated around the UTCHMMA and uniform operands stay in
-// uniform registers.  All 32 lanes must execute this (converged).
-__device__ __forceinline__ void mma_f16_elect_lh(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
-                                                 uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p, q;\n\t.reg .b64 da, db;\n\t"
-      "elect.sync _|q, 0xffffffff;\n\t"
-      "setp.ne.b32 p, %6, 0;\n\t"
-      "mov.b64 da, {%1, %2};\n\tmov.b64 db, {%3, %4};\n\t"
-      "@q tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n\t}"
-      ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 // FOUR MMAs of a host-built issue program in one instruction group: w.x .. w.w = (A offset | B offset << 16) in 16-byte
 // units relative to a_base / b_base, 0xffffffff = no MMA (padding of the program to a multiple of four).  One election
 // and one 128-bit constant load per four MMAs; the first MMA takes `accumulate_first`, the others accumulate.
+// (`elect.sync` inside the group tells ptxas that exactly one lane issues: no per-lane ELECT / BRA.U.ANY loop around the
+// UTCHMMA, uniform operands stay in uniform registers.  All 32 lanes must execute this, converged.)
 // (Measured on the one-word-per-iteration loop, ncu source view: ~105 issue cycles per MMA against 61 of tensor time -
 // the indexed constant load sat on the critical path of every MMA, plus ELECT / VOTEU / 4 x R2UR each.)
 __device__ __forceinline__ void mma_f16_x4(uint32_t d_tmem, uint32_t a_base, uint32_t a_hi, uint32_t b_base, uint32_t b_hi,
@@ -244,8 +211,8 @@ __device__ __forceinline__ void mma_commit(uint64_t* bar) {
                : "memory");
 }
 
-// commit issued by the SAME elected lane as mma_f16_elect_lh (elect.sync is deterministic for a given member mask): the
-// commit tracks the MMAs of the executing thread only.  Warp-converged.
+// commit issued by the SAME elected lane as the elect.sync issue groups above (elect.sync is deterministic for a given member
+// mask): the commit tracks the MMAs of the executing thread only.  Warp-converged.
 __device__ __forceinline__ void mma_commit_elect(uint64_t* bar) {
   asm volatile(
       "{\n\t.reg .pred q;\n\telect.sync _|q, 0xffffffff;\n\t"

@@ -410,7 +410,6 @@ class QuantConv2dFn(Function):
         L.require_cuda(x, wq)
         assert not (pre_relu and any(ctx.needs_input_grad)), "the folded ReLU is an inference-only fusion"
         lib = L.load()
-        packed = getattr(x, "_mnb_packed", None) if L.USE_PACKED else None   # experimental, see fused.BNSignFn
         x = x.contiguous()
         wq = wq.contiguous()
         sh = _shape_struct(x.shape, wq.shape, stride, padding, dilation, groups)
@@ -446,60 +445,22 @@ class QuantConv2dFn(Function):
         if (not done and L.PK_MODE != "off" and x.dtype == torch.float32 and (L.PK_MODE == "all" or spec is not None)
                 and not getattr(x, "_mnb_plane_only", False)):
             done = _pk_forward(ctx, x, wq, bias, w_int, w_scale, spec, sh, y, ctx.needs_input_grad[0], pre_relu=pre_relu)
-        pm1_plane = getattr(x, "_mnb_pk_pm1", None)
-        if (not done and L.PK_WBWTAB and L.PK_MODE != "off" and spec is None and w_int is not None and x.dtype == torch.float32
-                and getattr(x, "_mnb_pm1", False) and (pm1_plane is not None or sh.ker_h * sh.ker_w > 1)):
-            # wbwtab layer behind a fused BatchNorm + binarizer: +-1 input (one exact bf16 piece).  With the producer's plane
-            # the layer is pure TMA -> MMA; 3x3 layers win on the packed-operand family even when they pack themselves
-            # (measured per layer, DESIGN.md 6).  Falls through to the fused kernels when the shape is outside the cover.
-            if pm1_plane is not None and pm1_plane.numel() != x.numel() * 2:
-                pm1_plane = None
-            done = _pk_forward(ctx, x, wq, bias, w_int, w_scale, None, sh, y, ctx.needs_input_grad[0], prepacked=pm1_plane,
+        if (not done and L.PK_MODE != "off" and spec is None and x.dtype == torch.float32 and getattr(x, "_mnb_pm1", False)
+                and not pre_relu):
+            # conv behind a binarizer (a wbwtab layer, or with fp32 weights the 10-way head, fused.EnginePmConv2d): the +-1
+            # input is ONE exact bf16 piece.  With the plane a fused BatchNorm + binarizer wrote (fused.BNSignFn) the layer is
+            # pure TMA -> MMA, without it the layer packs its own input
+            plane = getattr(x, "_mnb_pk_pm1", None)
+            if plane is not None and plane.numel() != x.numel() * 2:
+                plane = None
+            done = _pk_forward(ctx, x, wq, bias, w_int, w_scale, None, sh, y, ctx.needs_input_grad[0], prepacked=plane,
                                pm1=True)
-        if (not done and L.PK_MODE != "off" and spec is None and w_int is None and x.dtype == torch.float32
-                and getattr(x, "_mnb_pm1", False) and not pre_relu):
-            # un-quantized conv behind a binarizer (the 10-way head of a wbwtab model, fused.EnginePmConv2d): the +-1 input is
-            # ONE exact bf16 piece - the producer's plane when it wrote one - against exact pieces of the fp32 weights
-            plane = pm1_plane if (pm1_plane is not None and pm1_plane.numel() == x.numel() * 2) else None
-            done = _pk_forward(ctx, x, wq, bias, None, None, None, sh, y, ctx.needs_input_grad[0], prepacked=plane, pm1=True)
         if not done and getattr(x, "_mnb_plane_only", False):
             x = materialized(x)   # outside the packed-operand cover (rare): the kernels below read the fp32 values
         if not done and pre_relu:
             x = torch.relu(x)     # outside the packed-operand cover: the folded ReLU as its own pass
-        if not done and packed is not None and spec is None and w_int is not None and packed.numel() == x.numel() \
-                and L.PK_MODE != "off" and sh.stride_h == 1:
-            # the BatchNorm + binarizer producer also wrote its +-1 output as the bf16 plane the packed-operand family
-            # reads (fused.BNSignFn): forward = TMA -> MMA -> epilogue on 2 B/element, no pack pass, no converter warps.
-            # The backward of this layer stays on the fused kernels below (they re-read the fp32 tensor).
-            from . import pk as PK
-            if PK.supported(sh, 0, 1, 1):
-                w_img = PK.pack_weight(sh, 0, 1, 1, w_int=w_int)
-                rc = _timed("fwd_pk", sh, lambda: PK.conv(sh, 0, packed, 1, w_img, 1, y, n_scale=w_scale, bias=bias))
-                if rc == 0:
-                    done = True
-                elif rc != L.E_UNSUPPORTED:
-                    L.check(rc, "pk_conv fwd (packed producer)")
-        if not done and L.USE_TC and w_int is not None and x.dtype == torch.float32:
-            # fused tcgen05 path: quantize inside the operand staging of the tensor-core conv
-            qp = None
-            if spec is not None:
-                qp = spec.struct()
-                codes = torch.empty(x.shape, dtype=torch.uint8, device=x.device)
-                if ctx.needs_input_grad[0]:
-                    bits = torch.zeros((x.numel() + 31) // 32, dtype=torch.int32, device=x.device)
-            wpack = torch.empty(w_int.numel(), dtype=torch.int16, device=x.device)
-            rc = _timed("fwd_tc", sh, lambda: lib.mnb_fq_conv2d_fwd_tc(
-                C.byref(sh), x.data_ptr(), None if qp is None else C.byref(qp), w_int.data_ptr(),
-                w_scale.data_ptr(), L.ptr(bias), y.data_ptr(), L.ptr(codes), L.ptr(bits), wpack.data_ptr(),
-                L.tc_err_flag(x.device).data_ptr(), L.stream()))
-            if rc == 0:
-                done = True
-            elif rc == L.E_UNSUPPORTED:
-                codes = bits = None
-            else:
-                L.check(rc, "fq_conv2d_fwd_tc")
         ctx.fconv = False
-        if not done and L.USE_TC and spec is None and x.dtype == torch.float32:
+        if not done and spec is None and x.dtype == torch.float32:
             # un-quantized input with few channels (first layer): fp32-accurate im2col conv on the tensor cores
             rc = _timed("fconv_fwd_tc", sh, lambda: lib.mnb_fconv2d_fwd_tc(
                 C.byref(sh), x.data_ptr(), wq.data_ptr(), L.ptr(bias), y.data_ptr(),
@@ -533,7 +494,7 @@ class QuantConv2dFn(Function):
                 a_scale = spec.scale
         ctx.sh, ctx.spec, ctx.a_scale = sh, spec, a_scale
         ctx.codes, ctx.bits = codes, bits
-        ctx.x = x if (not ctx.pk and (codes is None or (L.USE_TC and w_int is not None))) else None
+        ctx.x = x if (not ctx.pk and codes is None) else None   # fp32 input of the generic / tcfp32 weight gradient
         ctx.wq = wq
         ctx.w_int, ctx.w_scale = (w_int, w_scale) if w_int is not None else (None, None)
         ctx.has_bias = bias is not None
@@ -559,58 +520,27 @@ class QuantConv2dFn(Function):
             dx = torch.empty((sh.batch, sh.in_c, sh.in_h, sh.in_w), dtype=torch.float32, device=dy.device)
             qp = spec.struct() if spec is not None else None
             bits_ptr = ctx.bits.data_ptr() if spec is not None else None
-            rc = L.E_UNSUPPORTED
-            if L.USE_TC and ctx.w_int is not None:
-                wpack = torch.empty(ctx.w_int.numel(), dtype=torch.int16, device=dy.device)
-                rc = _timed("dgrad_tc", sh, lambda: lib.mnb_conv2d_dgrad_tc(
-                    C.byref(sh), dy.data_ptr(), ctx.w_int.data_ptr(), ctx.w_scale.data_ptr(), bits_ptr,
-                    None if qp is None else C.byref(qp), dx.data_ptr(), wpack.data_ptr(),
-                    L.tc_err_flag(dy.device).data_ptr(), L.stream()))
-            if rc == L.E_UNSUPPORTED:
-                rc = _timed("dgrad", sh, lambda: lib.mnb_conv2d_dgrad(
-                    C.byref(sh), dy.data_ptr(), ctx.wq.data_ptr(), bits_ptr, None if qp is None else C.byref(qp),
-                    dx.data_ptr(), L.stream()))
-            L.check(rc, "conv2d_dgrad")
+            L.check(_timed("dgrad", sh, lambda: lib.mnb_conv2d_dgrad(
+                C.byref(sh), dy.data_ptr(), ctx.wq.data_ptr(), bits_ptr, None if qp is None else C.byref(qp),
+                dx.data_ptr(), L.stream())), "conv2d_dgrad")
         if ctx.needs_input_grad[1]:
             dwq = torch.empty_like(ctx.wq)
-            ops = L.ConvOperands()
-            if ctx.codes is not None:
-                ops.a_codes = ctx.codes.data_ptr()
-                ops.a_offset = spec.code_offset
-                ops.a_offset_zp = L.ptr(spec.zero_point) if spec.mode == L.ACT_IAO else None
-                ops.a_scale = L.ptr(ctx.a_scale)
+            fbytes = int(lib.mnb_fconv2d_wgrad_tc_scratch_bytes(C.byref(sh))) if ctx.fconv else -1
+            if fbytes >= 0:
+                ws = torch.empty(max(fbytes, 4), dtype=torch.uint8, device=dy.device)
+                L.check(_timed("fconv_wgrad_tc", sh, lambda: lib.mnb_fconv2d_wgrad_tc(
+                    C.byref(sh), dy.data_ptr(), ctx.x.data_ptr(), dwq.data_ptr(), ws.data_ptr(),
+                    L.tc_err_flag(dy.device).data_ptr(), L.stream())), "fconv2d_wgrad_tc")
             else:
-                ops.a_f32 = ctx.x.data_ptr()
-            nbytes = int(lib.mnb_wgrad_scratch_bytes(C.byref(sh)))
-            done = False
-            if ctx.fconv:
-                fbytes = int(lib.mnb_fconv2d_wgrad_tc_scratch_bytes(C.byref(sh)))
-                if fbytes >= 0:
-                    ws = torch.empty(max(fbytes, 4), dtype=torch.uint8, device=dy.device)
-                    L.check(_timed("fconv_wgrad_tc", sh, lambda: lib.mnb_fconv2d_wgrad_tc(
-                        C.byref(sh), dy.data_ptr(), ctx.x.data_ptr(), dwq.data_ptr(), ws.data_ptr(),
-                        L.tc_err_flag(dy.device).data_ptr(), L.stream())), "fconv2d_wgrad_tc")
-                    done = True
-            if not done and L.USE_TC and ctx.w_int is not None and ctx.x is not None:
-                tbytes = int(lib.mnb_wgrad_tc_scratch_bytes(C.byref(sh)))
-                if tbytes > 0:
-                    qp = spec.struct() if spec is not None else None
-                    ws = torch.empty(max(tbytes, nbytes, 4), dtype=torch.uint8, device=dy.device)
-                    inexact = torch.zeros(1, dtype=torch.int32, device=dy.device)
-                    rc = _timed("wgrad_tc", sh, lambda: lib.mnb_conv2d_wgrad_tc(
-                        C.byref(sh), dy.data_ptr(), ctx.x.data_ptr(), None if qp is None else C.byref(qp),
-                        dwq.data_ptr(), ws.data_ptr(), inexact.data_ptr(), L.tc_err_flag(dy.device).data_ptr(),
-                        L.stream()))
-                    if rc == 0:
-                        done = True
-                        if spec is None:
-                            # raw fp32 activations that are not bf16-exact: device-side fallback, no host sync
-                            L.check(lib.mnb_conv2d_wgrad_cond(C.byref(sh), dy.data_ptr(), C.byref(ops), dwq.data_ptr(),
-                                                              ws.data_ptr(), inexact.data_ptr(), L.stream()),
-                                    "conv2d_wgrad_cond")
-                    elif rc != L.E_UNSUPPORTED:
-                        L.check(rc, "conv2d_wgrad_tc")
-            if not done:
+                ops = L.ConvOperands()
+                if ctx.codes is not None:
+                    ops.a_codes = ctx.codes.data_ptr()
+                    ops.a_offset = spec.code_offset
+                    ops.a_offset_zp = L.ptr(spec.zero_point) if spec.mode == L.ACT_IAO else None
+                    ops.a_scale = L.ptr(ctx.a_scale)
+                else:
+                    ops.a_f32 = ctx.x.data_ptr()
+                nbytes = int(lib.mnb_wgrad_scratch_bytes(C.byref(sh)))
                 ws = torch.empty(max(nbytes, 4), dtype=torch.uint8, device=dy.device)
                 L.check(_timed("wgrad", sh, lambda: lib.mnb_conv2d_wgrad(
                     C.byref(sh), dy.data_ptr(), C.byref(ops), dwq.data_ptr(), ws.data_ptr(), L.stream())),

@@ -49,8 +49,8 @@ class BNSignFn(Function):
                                              L.stream()), "bn_sign_pool_fwd")
         else:
             y = torch.empty_like(x)
-            packed = None
-            if L.PK_WBWTAB and not L.USE_PACKED and c % 8 == 0 and hw % 32 == 0 and x.dim() == 4 and L.PK_MODE != "off":
+            rc = L.E_UNSUPPORTED
+            if c % 8 == 0 and hw % 32 == 0 and x.dim() == 4 and L.PK_MODE != "off":
                 # the +-1 output also as the operand plane of the consuming conv (packed-operand family): 2 extra bytes per
                 # element here save that conv's 4-byte read and its pack pass
                 plane = torch.empty(x.numel() * 2, dtype=torch.uint8, device=x.device)
@@ -64,25 +64,12 @@ class BNSignFn(Function):
                     y._mnb_pk_pm1 = plane
                     if skip_y:
                         y._mnb_plane_only = True    # functional.materialized(y) rebuilds the values from the plane
-                    packed = False          # done (not the experimental bf16 tensor of MNB_PACKED_OPERANDS)
                 elif rc != L.E_UNSUPPORTED:
                     L.check(rc, "bn_sign_fwd_packed")
-            if packed is None and L.USE_PACKED and c % 8 == 0 and hw % 32 == 0:
-                # experimental (MNB_PACKED_OPERANDS=1): also emit the bf16 position-major operand of the next conv
-                packed = torch.empty(x.numel(), dtype=torch.bfloat16, device=x.device)
-                rc = lib.mnb_bn_sign_fwd_packed(x.data_ptr(), b, c, hw, mean.data_ptr(), invstd.data_ptr(), gamma.data_ptr(),
-                                                beta.data_ptr(), shuffle_groups, y.data_ptr(), bits.data_ptr(),
-                                                packed.data_ptr(), L.stream())
-                if rc == L.E_UNSUPPORTED:
-                    packed = None
-                else:
-                    L.check(rc, "bn_sign_fwd_packed")
-            if packed is None:
+            if rc != 0:
                 L.check(lib.mnb_bn_sign_fwd(x.data_ptr(), b, c, hw, mean.data_ptr(), invstd.data_ptr(), gamma.data_ptr(),
                                             beta.data_ptr(), shuffle_groups, y.data_ptr(), bits.data_ptr(), L.stream()),
                         "bn_sign_fwd")
-            elif packed is not False:
-                y._mnb_packed = packed   # picked up by QuantConv2dFn.forward when y is its input
         y._mnb_pm1 = True        # exactly +-1: a consuming conv may pack it as ONE bf16 piece
         ctx.save_for_backward(x, gamma, mean, invstd)
         ctx.bits, ctx.arg, ctx.training, ctx.shuffle_groups = bits, arg, training, shuffle_groups
@@ -103,7 +90,7 @@ class BNSignFn(Function):
         dgamma, dbeta, dx_sum = out[:c], out[c:2 * c], out[2 * c:]
         scratch = L.scratch(x.device, c)
         if (ctx.arg is not None and ctx.pk_conv is not None and ctx.training and c % 8 == 0 and x.shape[3] % 8 == 0
-                and x.shape[2] % 2 == 0 and "mnb_bn_sign_pool_bwd_pack" in L.PROTOTYPES):
+                and x.shape[2] % 2 == 0):
             # pooled producer behind a conv of the packed-operand family: reduce pass (dgamma, dbeta), then the apply pass
             # writes the full-resolution gradient straight as that conv's packed operand (no fp32 dx, no pack pass)
             w_scale, T = ctx.pk_conv
@@ -124,7 +111,7 @@ class BNSignFn(Function):
                                              1 if ctx.training else 0, ctx.shuffle_groups, dx.data_ptr(), dgamma.data_ptr(),
                                              dbeta.data_ptr(), dx_sum.data_ptr(), scratch.data_ptr(), L.stream()),
                     "bn_sign_pool_bwd")
-        elif ctx.pk_conv is not None and ctx.training and c % 8 == 0 and "mnb_bn_sign_bwd_pack" in L.PROTOTYPES:
+        elif ctx.pk_conv is not None and ctx.training and c % 8 == 0:
             # reduce pass of mnb_bn_sign_bwd (dgamma, dbeta), then the apply pass that writes dx as the producing conv's packed
             # gradient operand.  The channel sums of dx (that conv's bias gradient) are exactly zero behind a training-mode
             # BatchNorm; the reference's value is the rounding noise of that sum.

@@ -1,7 +1,8 @@
 """Python side of the packed-operand tensor-core family (``csrc/mnb_pk.cu``).
 
-Every conv of the QAT models that the fused kernels of ``mnb_conv_tc_*.cu`` cannot take (weights that do not fit in
-shared memory, stride 2, 5x5 filters, 4x4 or 224x224 images ...) and every fused-quantizer layer runs here:
+Every quantized conv of the QAT models runs here, from 1x1 grouped layers to ResNet-18's 512 -> 512 3x3 layers (weights
+streamed, stride 2, 5x5 filters, 4x4 or 224x224 images); only the fp32 first layer (``mnb_conv_fp32_tc.cu``) and shapes
+outside the cover (functional.QuantConv2dFn falls through to the generic kernels) do not:
 
     pack_act    fp32 NCHW -> bf16 term planes [t][b][c/8][h][w][8] (fake-quantize, or exact split of an fp32 tensor)
     pack_weight integer levels / fp32 weights -> the bf16 operand image of one (shape, mode)

@@ -253,7 +253,7 @@ def test_dorefa_fuse_option_agrees_with_the_unfused_engine():
 def test_wbwtab_layer_between_two_fused_producers_on_the_packed_operand_family(cfg, pool):
     """BatchNormBinarize2d -> wbwtab QuantConv2d -> BatchNormBinarize2d with both conv operands written by the producers
     (+-1 plane forward: mnb_bn_sign_fwd_packed, gradient pieces backward: mnb_bn_sign_bwd_pack) against the same chain on the
-    fused kernels (MNB_PK_WBWTAB=0), which the oracle tests pin: identical +-1 outputs, gradients to 1e-5 (weight gradient:
+    generic kernels (MNB_PK=off), which the oracle tests pin: identical +-1 outputs, gradients to 1e-5 (weight gradient:
     plus the cancellation allowance of tests/test_gpu_parity.py).  ``pool``: the consuming producer has the 2x2 max-pool folded
     in (mnb_bn_sign_pool_bwd_pack writes the full-resolution gradient pieces)."""
     import micronet_b200 as E
@@ -267,8 +267,8 @@ def test_wbwtab_layer_between_two_fused_producers_on_the_packed_operand_family(c
     bn0, bn1 = _pair(C, 3), _pair(K, 4)
     conv = E.wbwtab.QuantConv2d(C, K, R, padding=R // 2, groups=G, W=3)
     res = {}
-    for mode in (False, True):
-        L.PK_WBWTAB = mode
+    for mode in ("off", "auto"):
+        L.PK_MODE = mode
         try:
             p0 = BatchNormBinarize2d(C); p0.load_state_dict(bn0.state_dict()); p0.out_shuffle_groups = sg
             p1 = BatchNormBinarize2d(K); p1.load_state_dict(bn1.state_dict()); p1.pool2 = pool
@@ -283,8 +283,8 @@ def test_wbwtab_layer_between_two_fused_producers_on_the_packed_operand_family(c
             res[mode] = dict(out=out.detach().cpu(), conv=captured["y"].cpu(), dx=xg.grad.cpu(), dw=cv.weight.grad.cpu(),
                              db=cv.bias.grad.cpu(), dg1=p1.weight.grad.cpu(), db1=p1.bias.grad.cpu(), dg0=p0.weight.grad.cpu())
         finally:
-            L.PK_WBWTAB = True
-    a, b = res[False], res[True]
+            L.PK_MODE = "auto"
+    a, b = res["off"], res["auto"]
     assert rel_err(b["conv"], a["conv"]) <= 1e-6                      # integer-level products: exact up to the bias add
     flips = (a["out"] != b["out"]).float().mean().item()
     assert flips <= 1e-4, flips                                         # sign of bn values within rounding of 0
@@ -364,3 +364,79 @@ def test_plane_only_producer_gives_the_same_block(shape):
     L.tc_check()
     for a, b in zip(res[True], res[False]):
         assert torch.equal(a, b)
+
+
+# B, C, H, W, K, R, groups, shuffle groups of the producer
+PLANE_CASES = [(4, 256, 32, 32, 256, 1, 2, 1), (4, 256, 32, 32, 256, 1, 2, 2), (4, 512, 16, 16, 512, 1, 4, 16),
+               (5, 1024, 8, 8, 1024, 1, 8, 32), (4, 256, 16, 16, 512, 3, 16, 2), (4, 512, 8, 8, 1024, 3, 32, 4),
+               (3, 64, 16, 16, 32, 3, 1, 1)]
+
+
+@pytest.mark.parametrize("case", PLANE_CASES, ids=[str(c) for c in PLANE_CASES])
+def test_packed_producer_and_conv_match_the_unpacked_path(case):
+    """The producer's bf16 operand plane (y._mnb_pk_pm1, mnb_bn_sign_fwd_packed) is exactly the +-1 output in
+    [B][C/8][H][W][8] order (the producer's OUTPUT channel order), and the convolution fed by it equals an fp64 convolution
+    of the fp32 tensor."""
+    import torch.nn.functional as TF
+    from micronet_b200 import _lib as L, functional as F_
+    from micronet_b200.fused import BatchNormBinarize2d
+    B, C, H, W, K, R, G, sg = case
+    torch.manual_seed(sum(case))
+    bn = BatchNormBinarize2d(C).to(DEV).train()
+    bn.out_shuffle_groups = sg
+    with torch.no_grad():
+        bn.weight.copy_(torch.rand(C) + 0.5)
+        bn.bias.copy_(torch.randn(C) * 0.3)
+    x = (torch.randn(B, C, H, W) * 1.5).to(DEV)
+    y = bn(x)
+    plane = getattr(y, "_mnb_pk_pm1", None)
+    assert plane is not None, "producer did not emit the packed operand"
+    want = y.detach().view(B, C // 8, 8, H, W).permute(0, 1, 3, 4, 2).contiguous().to(torch.bfloat16).flatten()
+    assert torch.equal(plane.view(torch.bfloat16), want)
+    w_int = torch.randint(-1, 2, (K, C // G, R, R), dtype=torch.int16).to(DEV)
+    w_scale = (torch.rand(K) * 0.02 + 0.001).to(DEV)
+    bias = torch.randn(K).to(DEV)
+    wq = w_int.float() * w_scale.view(-1, 1, 1, 1)
+    out = F_.quant_conv2d(y, wq, bias, w_int, w_scale, None, (1, 1), (R // 2, R // 2), (1, 1), G)
+    L.tc_check()
+    ref = TF.conv2d(y.detach().double().cpu(), wq.double().cpu(), bias.double().cpu(), 1, R // 2, 1, G)
+    assert rel_err(out.detach(), ref) < 2e-6
+
+
+@pytest.mark.parametrize("case", PLANE_CASES[:5], ids=[str(c) for c in PLANE_CASES[:5]])
+def test_block_with_packed_forward_has_the_same_gradients(case):
+    """BatchNorm+binarizer -> conv on the packed-operand family with producer-written operands (the default) against the
+    generic kernels (MNB_PK=off).  Same +-1 operand in the forward: identical outputs; gradients agree to the accuracy of the
+    backward's operand split."""
+    from micronet_b200 import _lib as L, functional as F_
+    from micronet_b200.fused import BatchNormBinarize2d
+    B, C, H, W, K, R, G, sg = case
+    torch.manual_seed(sum(case) + 1)
+    x0 = (torch.randn(B, C, H, W) * 1.5).to(DEV)
+    w_int = torch.randint(-1, 2, (K, C // G, R, R), dtype=torch.int16).to(DEV)
+    w_scale = (torch.rand(K) * 0.02 + 0.001).to(DEV)
+    go = torch.randn(B, K, H, W).to(DEV)
+    res = {}
+    for mode in ("off", "auto"):
+        L.PK_MODE = mode
+        try:
+            torch.manual_seed(5)
+            bn = BatchNormBinarize2d(C).to(DEV).train()
+            bn.out_shuffle_groups = sg
+            x = x0.clone().requires_grad_(True)
+            wq = (w_int.float() * w_scale.view(-1, 1, 1, 1)).requires_grad_(True)
+            F_.TIMER = F_.KernelTimer()
+            out = F_.quant_conv2d(bn(x), wq, None, w_int, w_scale, None, (1, 1), (R // 2, R // 2), (1, 1), G)
+            out.backward(go)
+            torch.cuda.synchronize()
+            kinds = {k for k, _, _, _ in F_.TIMER.records}
+            res[mode] = (out.detach(), x.grad, wq.grad, bn.weight.grad, kinds)
+        finally:
+            L.PK_MODE = "auto"
+            F_.TIMER = None
+    assert not any(k.endswith("_pk") for k in res["off"][4]), res["off"][4]
+    assert {"fwd_pk", "dgrad_pk", "wgrad_pk"} <= res["auto"][4], res["auto"][4]
+    assert rel_err(res["auto"][0], res["off"][0]) <= 1e-6
+    for a, b in zip(res["auto"][1:4], res["off"][1:4]):
+        assert rel_err(a, b) <= 1e-5     # two-piece dy operand (MNB_PK_TERMS_BWD=2): ~3e-6, inside the 1e-5 contract
+    L.tc_check()

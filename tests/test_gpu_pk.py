@@ -31,6 +31,12 @@ SHAPES = [
     (1, 3, 64, 64, 16, 7, 2, 3, 1),       # 7x7 stride-2 stem
     (2, 32, 9, 9, 48, 3, 1, 0, 1),        # 'valid' padding, odd size
     (9, 512, 1, 1, 10, 1, 1, 0, 1),       # linear layer view
+    (4, 512, 16, 16, 512, 1, 1, 0, 4),    # NIN-GC grouped 1x1, 4 groups
+    (4, 512, 8, 8, 1024, 3, 1, 1, 32),    # NIN-GC grouped 3x3, 32 groups
+    (5, 1024, 8, 8, 1024, 1, 1, 0, 8),    # NIN-GC grouped 1x1, 8 groups, odd batch
+    (3, 48, 4, 4, 64, 1, 1, 0, 1),        # 4x4 images, 1x1
+    (2, 16, 12, 12, 16, 3, 1, 1, 1),      # W not a power of two
+    (2, 32, 16, 16, 32, 5, 1, 2, 1),      # 5x5, 32 channels
 ]
 IDS = ["x".join(map(str, s)) for s in SHAPES]
 

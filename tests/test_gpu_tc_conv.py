@@ -1,5 +1,5 @@
-"""Fused tcgen05 forward conv (mnb_fq_conv2d_fwd_tc) against the generic kernels, the standalone
-quantizer kernel (codes / STE bits must be identical) and ATen-CPU conv2d."""
+"""QuantConv2dFn's default dispatch (the tensor-core kernels) against the generic CUDA-core kernels (MNB_PK=off) and
+ATen-CPU conv2d: forward, data gradient and weight gradient of the NIN-GC / NIN / ResNet layer shapes."""
 import numpy as np
 import pytest
 import torch
@@ -25,16 +25,17 @@ SHAPES = [
 ]
 
 
-def _run(x, wq, bias, w_int, w_scale, spec, R, G, use_tc):
+def _run(x, wq, bias, w_int, w_scale, spec, R, G, pk_mode, pm1):
     from micronet_b200 import _lib as L, functional as F_
-    L.USE_TC = use_tc
+    L.PK_MODE = pk_mode
     try:
         xg = x.clone().requires_grad_(True)
+        xg._mnb_pm1 = pm1     # +-1 input (a binarizer's output without a producer-written plane)
         y = F_.quant_conv2d(xg, wq, bias, w_int, w_scale, spec, (1, 1), (R // 2, R // 2), (1, 1), G)
         torch.cuda.synchronize()
         return y
     finally:
-        L.USE_TC = True
+        L.PK_MODE = "auto"
 
 
 @pytest.mark.parametrize("shape", SHAPES, ids=[str(s) for s in SHAPES])
@@ -72,9 +73,9 @@ def test_tc_forward_matches_generic_and_cpu(shape, mode):
     err = L.tc_err_flag(torch.device(DEV))
     err.zero_()
     n0 = L.launch_count()
-    y_tc = _run(xd, wqd, bd, wid, wsd, spec, R, G, True)
+    y_tc = _run(xd, wqd, bd, wid, wsd, spec, R, G, "auto", mode == "raw_pm1")
     assert err.item() == 0, f"tensor-core pipeline timed out, code {err.item()}"
-    y_gen = _run(xd, wqd, bd, wid, wsd, spec, R, G, False)
+    y_gen = _run(xd, wqd, bd, wid, wsd, spec, R, G, "off", mode == "raw_pm1")
     assert torch.isfinite(y_tc).all()
     # both paths are exact on integer levels; on raw fp32 they differ only by fp32 summation order
     assert rel_err(y_tc, y_gen) <= (5e-6 if mode == "raw_fp32" else 1e-6), f"tc vs generic {rel_err(y_tc, y_gen)}"
@@ -88,47 +89,10 @@ def test_tc_forward_matches_generic_and_cpu(shape, mode):
     assert rel_err(y_tc, want) <= 1e-5, f"tc vs cpu {rel_err(y_tc, want)}"
 
 
-@pytest.mark.parametrize("shape", SHAPES[:5] + SHAPES[6:8], ids=str)
-@pytest.mark.parametrize("mode", ["dorefa8", "iao_sym"])
-def test_tc_forward_emits_identical_codes_and_bits(shape, mode):
-    import ctypes as C
-    from micronet_b200 import _lib as L, functional as F_
-    lib = L.load()
-    B, Cc, H, W, K, R, G = shape
-    g = torch.Generator().manual_seed(7)
-    x = (torch.randn(B, Cc, H, W, generator=g) * 4).to(DEV)
-    w_int = torch.randint(-127, 128, (K, Cc // G, R, R), generator=g, dtype=torch.int16).to(DEV)
-    w_scale = (torch.rand(K, generator=g) * 0.02 + 0.001).to(DEV)
-    if mode == "dorefa8":
-        spec = F_.ActSpec(L.ACT_DOREFA, bits=8)
-    else:
-        bufs = dict(scale=torch.tensor([9.0 / 127.5]), zero_point=torch.zeros(1), obs_min=torch.tensor([-9.0]),
-                    obs_max=torch.tensor([7.0]))
-        spec = F_.ActSpec(L.ACT_IAO, qmin=-128, qmax=127, q_type=0, **{k: v.to(DEV) for k, v in bufs.items()})
-    codes_ref, bits_ref, _ = F_.act_quant_raw(x, spec, True, True, False)
-    sh = L.ConvShape(B, Cc, H, W, K, R, R, 1, 1, R // 2, R // 2, 1, 1, G)
-    y = torch.empty(B, K, H, W, device=DEV)
-    codes = torch.full(x.shape, 77, dtype=torch.uint8, device=DEV)
-    bits = torch.zeros_like(bits_ref)
-    err = L.tc_err_flag(torch.device(DEV)); err.zero_()
-    qp = spec.struct()
-    wpack = torch.empty(w_int.numel(), dtype=torch.int16, device=DEV)
-    rc = lib.mnb_fq_conv2d_fwd_tc(C.byref(sh), x.data_ptr(), C.byref(qp), w_int.data_ptr(), w_scale.data_ptr(), None,
-                                  y.data_ptr(), codes.data_ptr(), bits.data_ptr(), wpack.data_ptr(), err.data_ptr(),
-                                  L.stream())
-    if rc == L.E_UNSUPPORTED:
-        pytest.skip("geometry not covered by the tensor-core kernel")
-    L.check(rc, "fq_conv2d_fwd_tc")
-    torch.cuda.synchronize()
-    assert err.item() == 0
-    assert torch.equal(codes, codes_ref)
-    assert torch.equal(bits, bits_ref)
-
-
 @pytest.mark.parametrize("shape", SHAPES, ids=[str(s) for s in SHAPES])
 @pytest.mark.parametrize("mode", ["raw", "dorefa8", "iao_sym"])
 def test_tc_dgrad_matches_generic_and_cpu(shape, mode):
-    """dx through the tensor-core dgrad (weight scale folded into dy, exact 3-term split, fused STE)."""
+    """dx through the tensor-core data gradient (weight scale folded into dy, MNB_PK_TERMS_BWD pieces, fused STE)."""
     from micronet_b200 import _lib as L, functional as F_
     B, C, H, W, K, R, G = shape
     g = torch.Generator().manual_seed(hash((shape, mode, "dgrad")) % (1 << 31))
@@ -147,18 +111,18 @@ def test_tc_dgrad_matches_generic_and_cpu(shape, mode):
     go = torch.randn(B, K, H, W, generator=g)
     err = L.tc_err_flag(torch.device(DEV)); err.zero_()
     grads = {}
-    for use_tc in (True, False):
-        L.USE_TC = use_tc
+    for pk_mode in ("auto", "off"):
+        L.PK_MODE = pk_mode
         try:
             xg = x.to(DEV).requires_grad_(True)
             y = F_.quant_conv2d(xg, wq.to(DEV), None, w_int.to(DEV), w_scale.to(DEV), spec, (1, 1), (R // 2, R // 2), (1, 1), G)
             y.backward(go.to(DEV))
             torch.cuda.synchronize()
-            grads[use_tc] = xg.grad.clone()
+            grads[pk_mode] = xg.grad.clone()
         finally:
-            L.USE_TC = True
+            L.PK_MODE = "auto"
     assert err.item() == 0, f"tensor-core pipeline timed out, code {err.item()}"
-    assert rel_err(grads[True], grads[False]) <= 5e-6, rel_err(grads[True], grads[False])  # fp32 summation order
+    assert rel_err(grads["auto"], grads["off"]) <= 5e-6, rel_err(grads["auto"], grads["off"])
     # CPU: autograd of conv2d on the dequantized input
     from oracle import reference_port as O
     xr = x.clone().requires_grad_(True)
@@ -172,14 +136,14 @@ def test_tc_dgrad_matches_generic_and_cpu(shape, mode):
         r = O._RoundRangeSTE.apply(v, torch.tensor([-9.0]) / s, torch.tensor([7.0]) / s, 0)
         xq = torch.clamp(r, -128, 127) * s
     TF.conv2d(xq, wq, None, 1, R // 2, 1, G).backward(go)
-    assert rel_err(grads[True], xr.grad) <= 1e-5, rel_err(grads[True], xr.grad)
+    assert rel_err(grads["auto"], xr.grad) <= 1e-5, rel_err(grads["auto"], xr.grad)
 
 
 @pytest.mark.parametrize("shape", SHAPES, ids=[str(s) for s in SHAPES])
 @pytest.mark.parametrize("mode", ["raw_pm1", "raw_fp32", "dorefa8", "iao_sym"])
 def test_tc_wgrad_matches_generic_and_cpu(shape, mode):
-    """dWq through the tensor-core wgrad (MN-major operands, TMEM-resident accumulators, deterministic
-    two-stage reduction); raw fp32 inputs that are not bf16-exact take the device-side fallback."""
+    """dWq through the tensor-core weight gradient (MN-major operands, deterministic reduction over the batch);
+    +-1 inputs are one exact bf16 piece, raw fp32 inputs MNB_PK_TERMS_BWD pieces."""
     from micronet_b200 import _lib as L, functional as F_
     from oracle import reference_port as O
     B, C, H, W, K, R, G = shape
@@ -202,19 +166,21 @@ def test_tc_wgrad_matches_generic_and_cpu(shape, mode):
     go = torch.randn(B, K, H, W, generator=g)
     err = L.tc_err_flag(torch.device(DEV)); err.zero_()
     grads = {}
-    for use_tc in (True, False):
-        L.USE_TC = use_tc
+    for pk_mode in ("auto", "off"):
+        L.PK_MODE = pk_mode
         try:
             wg = wq.to(DEV).requires_grad_(True)
-            y = F_.quant_conv2d(x.to(DEV), wg, None, w_int.to(DEV), w_scale.to(DEV), spec, (1, 1), (R // 2, R // 2), (1, 1), G)
+            xd = x.to(DEV)
+            xd._mnb_pm1 = mode == "raw_pm1"
+            y = F_.quant_conv2d(xd, wg, None, w_int.to(DEV), w_scale.to(DEV), spec, (1, 1), (R // 2, R // 2), (1, 1), G)
             y.backward(go.to(DEV))
             torch.cuda.synchronize()
-            grads[use_tc] = wg.grad.clone()
+            grads[pk_mode] = wg.grad.clone()
         finally:
-            L.USE_TC = True
+            L.PK_MODE = "auto"
     assert err.item() == 0, f"tensor-core pipeline timed out, code {err.item()}"
-    assert torch.isfinite(grads[True]).all()
-    assert rel_err(grads[True], grads[False]) <= 1e-5, rel_err(grads[True], grads[False])
+    assert torch.isfinite(grads["auto"]).all()
+    assert rel_err(grads["auto"], grads["off"]) <= 1e-5, rel_err(grads["auto"], grads["off"])
     if mode.startswith("raw"):
         xq = x
     elif mode == "dorefa8":
@@ -224,4 +190,4 @@ def test_tc_wgrad_matches_generic_and_cpu(shape, mode):
         xq = torch.clamp(O.round_half_away(x / s), -128, 127) * s
     wr = wq.clone().double().requires_grad_(True)
     TF.conv2d(xq.double(), wr, None, 1, R // 2, 1, G).backward(go.double())
-    assert rel_err(grads[True], wr.grad) <= 1e-5, rel_err(grads[True], wr.grad)
+    assert rel_err(grads["auto"], wr.grad) <= 1e-5, rel_err(grads["auto"], wr.grad)

@@ -5,7 +5,8 @@
   GPU run of round 2 (gpurun call r3g: 2 KB of extra static shared memory in `pk_conv_kernel`, `cudaFuncSetAttribute: invalid
   argument` on every launch);
 * the host-only plan of the packed-operand family (`mnb_pk_conv_plan`, `mnb_pk_wgrad_scratch_bytes`, `mnb_pk_wimage_bytes`,
-  `mnb_pk_act_bytes`) covers every convolution of the BASELINE.json models at their bench shapes, inside shared / tensor memory."""
+  `mnb_pk_act_bytes`) covers every convolution of the BASELINE.json models at their bench shapes, inside shared / tensor memory,
+  and every stride-1 layer with the operand pieces of a +-1 or raw fp32 input (functional.QuantConv2dFn's wbwtab layers)."""
 import ctypes as C
 import os
 import re
@@ -22,8 +23,6 @@ RESERVED = 1024             # per-block reservation that cuobjdump's SHARED figu
 BUDGETS = {
     "pk14pk_conv_kernel": ("mnb_pk.cu", "kSmemBudget"),
     "pk15pk_wgrad_kernel": ("mnb_pk.cu", "kSmemBudget"),
-    "tcconv14conv_tc_kernel": ("mnb_conv_tc_fwd.cu", "kMaxDynSmem"),
-    "tcwgrad15wgrad_tc_kernel": ("mnb_conv_tc_wgrad.cu", "kMaxDynSmem"),
     "tcfp3210fwd_kernel": ("mnb_conv_fp32_tc.cu", "kMaxDynSmem"),
     "tcfp3212wgrad_kernel": ("mnb_conv_fp32_tc.cu", "kMaxDynSmem"),
 }
@@ -107,3 +106,28 @@ def test_packed_operand_plan_covers_the_bench_models(conv):
     # plane sizes: one 16-byte vector per pixel and channel octet and piece
     assert int(lib.mnb_pk_act_bytes(B, Cc, H, W, 1)) == B * ((Cc + 7) // 8) * H * W * 16
     assert int(lib.mnb_pk_act_bytes(B, K, P, Q, Tb)) == Tb * B * ((K + 7) // 8) * P * Q * 16
+
+
+# B, C, H, W, K, R, groups (stride 1, 'same' padding): grouped NIN-GC layers, odd batch, 4x4 and 12x12 images, 5x5 filters
+STRIDE1_SHAPES = [
+    (4, 256, 32, 32, 256, 1, 2), (4, 256, 16, 16, 512, 3, 16), (4, 512, 16, 16, 512, 1, 4), (4, 512, 8, 8, 1024, 3, 32),
+    (5, 1024, 8, 8, 1024, 1, 8), (3, 192, 32, 32, 160, 1, 1), (2, 64, 32, 32, 64, 3, 1), (2, 32, 16, 16, 32, 5, 1),
+    (3, 48, 4, 4, 64, 1, 1), (2, 16, 12, 12, 16, 3, 1),
+]
+STRIDE1_CONVS = [("x".join(map(str, s)), s[0], s[1], s[2], s[3], s[4], s[5], 1, s[5] // 2, s[6]) for s in STRIDE1_SHAPES]
+STRIDE1_CONVS += [c for c in _model_convs() if c[7] == 1]
+
+
+@pytest.mark.parametrize("conv", STRIDE1_CONVS, ids=lambda c: c[0])
+def test_packed_operand_plan_covers_pm1_and_fp32_inputs(conv):
+    """forward with a +-1 (one piece), raw fp32 (PK_TERMS pieces) or asymmetric-IAO (two pieces) input against integer
+    weights, data gradient and weight gradient with the backward's pieces of dy and of the saved input"""
+    from micronet_b200 import _lib as L
+    lib = L.load()
+    name, B, Cc, H, W, K, R, st, pad, G = conv
+    sh = L.ConvShape(B, Cc, H, W, K, R, R, st, st, pad, pad, 1, 1, G)
+    Tb = min(L.PK_TERMS, L.PK_TERMS_BWD)
+    for mode, ta, tw in [(0, 1, 1), (0, 3, 1), (0, 2, 1), (1, Tb, 1)]:
+        assert lib.mnb_pk_conv_plan(C.byref(sh), mode, ta, tw, None) == 0, (name, mode, ta, tw, lib.mnb_last_error())
+    for tx in (1, Tb) if not name.startswith("res224") else ():   # configs[4] is inference only: no weight gradient at 224
+        assert int(lib.mnb_pk_wgrad_scratch_bytes(C.byref(sh), Tb, tx)) >= 0, (name, tx)
